@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- encoder images/sec at 1024^2 for the EV-M student (BASELINE.json metric), B200-native path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference|eager_gpu] [--batch B] [--img S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference|eager_gpu] [--batch B] [--img S] [--dump-outputs DIR]
 
 One "step" = one forward pass of the hot path over one synthetic batch (per GPU):
   ImageStudentEncoder(efficientvit_b1) : [B,3,S,S] fp32 NCHW -> [B,1024,E,E] fp32   (stage1/model.py:188-211)
@@ -18,6 +18,9 @@ Keys beyond the base contract: `roofline` (dominant kernel family by time, measu
 plus whole-step fractions and the top families), `cpu_baseline` (the oracle port timed on this box's host cores, rank 0, N=1),
 `e2e` (pinned host batch -> H2D -> module forward -> D2H of the step's scalar metric, every step), `also` (N=1: the other
 encoders, the teacher-embedding dump end to end with its real 85 MB/step D2H, and the PyTorch-eager GPU arm).
+`--dump-outputs DIR` (native) writes the embeddings of the last timed step, as the caller receives them, to DIR/embeddings.npy
+(fp32; above DUMP_MAX_ELEMS elements a fixed seeded sample of them, in flat-index order): the seeded weights and inputs are the
+same on every run with the same arguments, so two builds can be compared output for output.
 `--impl reference` times the CPU oracle port (the reference is Python/PyTorch; /root/reference does not exist on the GPU box,
 and the oracle is pinned to it by tests/golden) with all host threads.  `--impl eager_gpu` runs the same functional PyTorch
 restatement on the GPU -- the reference's eager CUDA path (cuDNN / cuBLAS), as shipped (TF32 + fp16 autocast) and strict fp32.
@@ -42,6 +45,17 @@ import torch  # noqa: E402
 
 METRIC = "encoder images/sec @1024^2 (EV-M student forward)"
 UNIT = "images/s"
+DUMP_MAX_ELEMS = 1 << 23          # 32 MB of fp32 per dumped array
+
+
+def dump_sample(t: torch.Tensor):
+    """`t` as fp32 numpy when it has at most DUMP_MAX_ELEMS elements, else the elements at a fixed seeded set of flat indices
+    (sorted): the same positions on every run for the same shape."""
+    t = t.detach()
+    if t.numel() > DUMP_MAX_ELEMS:
+        idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).unique()
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.float().cpu().numpy()
 
 
 def _peaks():
@@ -189,6 +203,11 @@ def run_native(args):
         launches = model.graph_launches_per_step * args.steps          # replayed from a CUDA graph: counted at capture
     ms_total = cx.max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        # now: with CUDA graphs `out` is the graph's output buffer, which later replays of the same input buffer overwrite
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "embeddings.npy"), dump_sample(out))
     ms_step = ms_total / args.steps
     value = world * B * args.steps / (ms_total / 1e3)
 
@@ -843,7 +862,13 @@ def main():
     ap.add_argument("--no-per-n", action="store_true", help="skip the per-N KD-step / teacher legs")
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="launch the eval plan kernel by kernel instead of replaying its CUDA graph")
     ap.add_argument("--table", default=None, help="write the per-kernel-family table (markdown) here")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the embeddings of the last timed step (rank 0; sampled above 32 MB) to DIR/embeddings.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs dumps the native path's outputs (--impl native)")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -63,7 +63,8 @@ def build(verbose: bool = False, force: bool = False) -> Path:
     with ThreadPoolExecutor(max_workers=min(8, max(1, len(jobs)))) as ex:
         list(ex.map(run, jobs))
     objs = [str(OBJ / (s.stem + ".o")) for s in srcs]
-    if jobs or force or not LIB.exists():
+    # relink when an object is newer than the library too: a build stopped between compiling and linking left it stale
+    if jobs or force or not LIB.exists() or any(os.path.getmtime(o) > LIB.stat().st_mtime for o in objs):
         tmp = LIB.with_suffix(".so.tmp")     # link beside the target, then rename: a reader never sees a half-written library
         run([nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", str(tmp), *objs, "-lcudart"])
         os.replace(tmp, LIB)

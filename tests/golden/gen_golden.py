@@ -333,7 +333,39 @@ def gen_sampler_cases():
     print("sampler_cases.json", len(cases), "cases")
 
 
+CONVERT_STUDENT = {"module.backbone.model.input_stem.op_list.0.conv.weight": 0.0, "student_trunk.head.0.weight": 1.0,
+                   "detector.backbone.vision_backbone.trunk.model.head.3.bias": 2.0, "head.1.running_mean": 3.0}
+CONVERT_SAM3 = {"detector.backbone.vision_backbone.trunk.blocks.0.attn.qkv.weight": 9.0,
+                "detector.backbone.vision_backbone.convs.0.conv_1x1.weight": 4.0, "detector.transformer.decoder.x": 5.0,
+                "tracker.sam_mask_decoder.y": 6.0, "detector.backbone.language_backbone.z": 7.0}
+CONVERT_SKIP = ["detector.backbone.language_backbone"]
+
+
+def gen_convert():
+    """The reference's stage1/convert_image_encoder_weights_stage1.py, run as a script on two tiny synthetic checkpoints
+    (one-element tensors) -> convert_merge.json: the inputs and the merged checkpoint's keys in order with their values."""
+    import json
+    import subprocess
+    import tempfile
+    script = os.path.join(install.REFERENCE_ROOT, "stage1", "convert_image_encoder_weights_stage1.py")
+    with tempfile.TemporaryDirectory() as tmp:
+        s, t, o = (os.path.join(tmp, n) for n in ("s.pth", "t.pth", "o.pth"))
+        torch.save({"model": {k: torch.full((1,), v) for k, v in CONVERT_STUDENT.items()}}, s)
+        torch.save({"model": {k: torch.full((1,), v) for k, v in CONVERT_SAM3.items()}}, t)
+        cmd = [sys.executable, script, "--student-ckpt", s, "--sam3-ckpt", t, "--output", o]
+        for p in CONVERT_SKIP:
+            cmd += ["--skip-teacher-prefix", p]
+        subprocess.run(cmd, check=True, capture_output=True)
+        merged = torch.load(o, weights_only=False)["model"]
+    rec = {"student": list(CONVERT_STUDENT.items()), "sam3": list(CONVERT_SAM3.items()), "skip_teacher_prefixes": CONVERT_SKIP,
+           "merged": [[k, float(v)] for k, v in merged.items()]}
+    json.dump(rec, open(os.path.join(HERE, "convert_merge.json"), "w"), indent=1)
+    print("convert_merge.json", len(rec["merged"]), "keys")
+
+
 def main(which):
+    if which in ("convert", "all"):
+        gen_convert()
     if which in ("sampler", "all"):
         gen_sampler_cases()
     if which in ("student_neck", "all"):
