@@ -108,6 +108,8 @@ SIGNATURES: dict[str, list] = {
     "es3_bilinear_bwd": [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp],
     "es3_litemla_attn_bwd_generic": [_vp, _ll, _vp, _ll, _vp, _i, _vp, _vp, _ll, _i, _i, _i, _i, _f, _vp],
     "es3_litemla_attn_bwd": [_vp, _ll, _vp, _ll, _vp, _i, _vp, _vp, _ll, _i, _i, _i, _f, _vp],
+    # input preprocessing (preprocess.cu)
+    "es3_preprocess_images": [_vp, _vp, _vp, _i, _i, _i, _vp, _vp],
 }
 
 # workspace-size helpers: name -> argtypes, restype long long

@@ -19,6 +19,7 @@ import torch.nn as nn
 
 from .. import ops
 from ..sam import MaskDecoder, PromptEncoder, TwoWayTransformer
+from ..stage1.transforms import ImagePreprocessor
 from .necks import Sam3DualViTDetNeck
 from .vitdet import create_sam3_vit_backbone
 
@@ -144,6 +145,7 @@ class SAM3InteractiveImagePredictor:
         self.model = sam_model
         self.mask_threshold = mask_threshold
         self.max_hole_area, self.max_sprinkle_area = max_hole_area, max_sprinkle_area
+        self._preprocess = None
         self.reset_predictor()
 
     @property
@@ -155,39 +157,41 @@ class SAM3InteractiveImagePredictor:
         self._orig_hw = None
         self.model._features = None
 
-    def _to_input(self, image):
-        """HWC uint8 ndarray / PIL image -> [3,S,S] fp32 on the device, resized and normalised like SAM2Transforms
-        (ToTensor -> Resize((S,S)) bilinear antialias -> Normalize(0.5, 0.5); sam1_utils.py:17-41).  Image decoding and
-        resizing are input plumbing outside the hot path and use torch."""
+    def _to_inputs(self, images):
+        """HWC uint8 / float ndarrays or PIL images -> ([B,3,S,S] fp32 on the device, [(h, w), ...]), resized and normalised like
+        SAM2Transforms (ToTensor -> Resize((S,S)) bilinear antialias -> Normalize(0.5, 0.5); sam1_utils.py:17-41) by one
+        es3_preprocess_images call for the whole list.  ToTensor leaves float arrays unscaled: they are taken as [0, 1]."""
         import numpy as np
-        arr = np.asarray(image)
-        if arr.ndim != 3 or arr.shape[2] != 3:
-            raise NotImplementedError("Image format not supported")
-        x = torch.from_numpy(np.ascontiguousarray(arr)).to(self.device).permute(2, 0, 1).float()
-        if arr.dtype == np.uint8:
-            x = x / 255.0
-        S = self.model.image_size
-        x = torch.nn.functional.interpolate(x[None], size=(S, S), mode="bilinear", align_corners=False, antialias=True)[0]
-        return (x - 0.5) / 0.5, tuple(arr.shape[:2])
+        arrs = []
+        for image in images:
+            arr = np.asarray(image)
+            if arr.ndim != 3 or arr.shape[2] != 3:
+                raise NotImplementedError("Image format not supported")
+            arrs.append(arr)
+        if self._preprocess is None:
+            S = self.model.image_size
+            self._preprocess = ImagePreprocessor(S, (127.5,) * 3, (127.5,) * 3, square=True, float_scale=255.0, device=self.device)
+        x, _ = self._preprocess(arrs)
+        return x, [tuple(a.shape[:2]) for a in arrs]
+
+    def _to_input(self, image):
+        """One image -> ([3,S,S] fp32 on the device, (h, w)); see _to_inputs."""
+        x, hw = self._to_inputs([image])
+        return x[0], hw[0]
 
     @torch.no_grad()
     def set_image(self, image):
         self.reset_predictor()
-        x, hw = self._to_input(image)
-        self._orig_hw = [hw]
-        self.model.set_image_batch(x[None])
+        x, self._orig_hw = self._to_inputs([image])
+        self.model.set_image_batch(x)
         self._is_image_set = True
 
     @torch.no_grad()
     def set_image_batch(self, image_list):
         self.reset_predictor()
         assert isinstance(image_list, list)
-        xs, self._orig_hw = [], []
-        for im in image_list:
-            x, hw = self._to_input(im)
-            xs.append(x)
-            self._orig_hw.append(hw)
-        self.model.set_image_batch(torch.stack(xs, dim=0))
+        x, self._orig_hw = self._to_inputs(image_list)
+        self.model.set_image_batch(x)
         self._is_image_set = self._is_batch = True
 
     def get_image_embedding(self):

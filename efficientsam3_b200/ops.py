@@ -47,7 +47,7 @@ class strict_precision:
 
 # ------------------------------------------------------------------------------------ accounting
 # kernels launched per C-ABI call (memsets excluded) -- bench.py reports the sum as `gpu_launches`.
-KERNELS_PER_CALL = {"es3_colsum_f32": 2, "es3_layernorm_bwd": 2, "es3_litemla_attn": 2, "es3_litemla_attn_generic": 2, "es3_fill_small_components": 4, "es3_grad_norm": 2, "es3_adamw_flat": 2, "es3_litemla_attn_tc": 2, "es3_kd_loss_fwd": 2, "es3_channel_mean": 2}
+KERNELS_PER_CALL = {"es3_colsum_f32": 2, "es3_layernorm_bwd": 2, "es3_litemla_attn": 2, "es3_litemla_attn_generic": 2, "es3_fill_small_components": 4, "es3_grad_norm": 2, "es3_adamw_flat": 2, "es3_litemla_attn_tc": 2, "es3_kd_loss_fwd": 2, "es3_channel_mean": 2, "es3_preprocess_images": 2}
 launch_count = 0
 
 
@@ -507,6 +507,25 @@ def cast_f32_to_f16(x, out=None):
         out = torch.empty(x.shape, device=x.device, dtype=torch.float16)
     assert out.is_cuda and out.dtype == torch.float16 and out.is_contiguous() and out.numel() == x.numel()
     _call("es3_cast_f32_to_f16", "cast_f32_f16", x.numel() * 6, 0, x.data_ptr(), out.data_ptr(), x.numel(), _stream())
+    return out
+
+
+def preprocess_images(table, affine, S, max_out, taps_floats, in_bytes, out=None):
+    """Resize + normalise + pad a batch of decoded images into out [B,3,S,S] fp32 (es3_preprocess_images).  table [B,16] int64
+    and affine [B,6] fp32 are CUDA tensors as stage1.transforms.build_table lays them out; `in_bytes` (the images' bytes) is
+    for the profiler.  `out` may be a preallocated buffer (a loader rotating the inputs of a graphed encoder)."""
+    _chk(table, torch.int64, "table"); _chk(affine, torch.float32, "affine")
+    _ensure_init(table)
+    B = table.shape[0]
+    assert table.shape == (B, 16) and affine.shape == (B, 6) and table.is_contiguous() and affine.is_contiguous()
+    if out is None:
+        out = torch.empty((B, 3, S, S), device=table.device, dtype=torch.float32)
+    _chk(out, torch.float32, "out")
+    if tuple(out.shape) != (B, 3, S, S) or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous [{B},3,{S},{S}] fp32 tensor, got {tuple(out.shape)}")
+    taps = torch.empty(max(int(taps_floats), 1), device=table.device, dtype=torch.float32)
+    _call("es3_preprocess_images", "preprocess", int(in_bytes) + _nb(out), 0, table.data_ptr(), affine.data_ptr(), taps.data_ptr(),
+          B, S, max_out, out.data_ptr(), _stream())
     return out
 
 

@@ -217,10 +217,12 @@ class EmbeddingDumper:
 
 
 @torch.no_grad()
-def save_embeddings_one_epoch(model, data_loader, path: str, rank: int = 0, max_batch: int | None = None):
+def save_embeddings_one_epoch(model, data_loader, path: str, rank: int = 0, max_batch: int | None = None, preprocess=None):
     """Native counterpart of save_embeddings_one_epoch (save_embedding_image_stage1.py:69-126).
     `data_loader` yields ((samples, _), (keys, seeds)) with `samples` a list/tensor of [3,S,S] fp32 images, exactly what the
-    reference's write-mode DatasetWrapper + pseudo_collate produce.  Returns the number of records written."""
+    reference's write-mode DatasetWrapper + pseudo_collate produce.  With `preprocess` (a stage1.transforms.ImagePreprocessor)
+    `samples` are decoded images of any size, resized, normalised and padded on the device.  Returns the number of records
+    written."""
     model.eval()
     dev = next(model.parameters()).device
     dumper = None
@@ -228,8 +230,11 @@ def save_embeddings_one_epoch(model, data_loader, path: str, rank: int = 0, max_
     with EmbeddingStoreWriter(path, rank) as writer:
         try:
             for (samples, _), (keys, seeds) in data_loader:
-                x = samples if torch.is_tensor(samples) else torch.stack(list(samples), dim=0)
-                x = x.to(dev, non_blocking=True)
+                if preprocess is not None:
+                    x, _ = preprocess(list(samples))
+                else:
+                    x = samples if torch.is_tensor(samples) else torch.stack(list(samples), dim=0)
+                    x = x.to(dev, non_blocking=True)
                 out = model(x)
                 if dumper is None:
                     cap = (max_batch or getattr(data_loader, "batch_size", None) or x.shape[0]) * out[0].numel()

@@ -20,10 +20,12 @@ def set_bn_state(config, model):
                 m.eval()
 
 
-def train_one_epoch(config, model, data_loader, optimizer, epoch, lr_at=None, on_step=None):
+def train_one_epoch(config, model, data_loader, optimizer, epoch, lr_at=None, on_step=None, preprocess=None):
     """One epoch of stage-1 distillation.  `optimizer`: stage1.optim.FlatAdamW over `model`.  `lr_at(update_index) -> lr`
     replaces `lr_scheduler.step_update` (default: the reference's cosine schedule built from config.TRAIN).  `on_step(idx, loss)`
     is called after every iteration with the detached device loss (call `.item()` there only when you log: it syncs).
+    `preprocess`: a stage1.transforms.ImagePreprocessor; `samples` are then decoded images of any size, resized, normalised
+    and padded on the device, and img_size_before_pad comes from it.
     Returns the list of per-iteration losses (device scalars)."""
     model.train()
     set_bn_state(config, model)
@@ -55,11 +57,14 @@ def train_one_epoch(config, model, data_loader, optimizer, epoch, lr_at=None, on
     dev = next(model.parameters()).device
     losses = []
     for idx, ((samples, annos), (saved_embeddings, seeds)) in enumerate(data_loader):
-        samples = torch.stack(list(samples), dim=0).to(dev, non_blocking=True)
+        if preprocess is not None:
+            samples, sizes = preprocess(list(samples))
+        else:
+            samples, sizes = torch.stack(list(samples), dim=0).to(dev, non_blocking=True), annos["img_size_before_pad"]
         saved = torch.from_numpy(np.stack(saved_embeddings, axis=0)).float()
         saved = saved.view(samples.size(0), *embed_shape).to(dev, non_blocking=True)
         update = (idx + 1) % accum == 0
-        loss = kd_train_step(model, optimizer, samples, saved, annos["img_size_before_pad"], cosine_weight=cosine_w,
+        loss = kd_train_step(model, optimizer, samples, saved, sizes, cosine_weight=cosine_w,
                              clip_grad=config.TRAIN.CLIP_GRAD, lr=lr_for_update(idx) if update else None,
                              accumulation_steps=accum, update=update)
         losses.append(loss)

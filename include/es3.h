@@ -424,6 +424,19 @@ int es3_attention_f32(const float* qkv, float* out, const float* bias, const flo
                       int head_dim, int q_off, int k_off, int v_off, int head_stride, int win, float scale, void* stream);
 int es3_scale_channels_f32(const float* x, const float* gate, float* y, int B, long long HW, int C, void* stream);
 
+/* ------------------------------------------------------------------------------------------ input preprocessing */
+/* Decoded images of any size -> antialiased bilinear resize (torch's _upsample_bilinear2d_aa, align_corners=False: width pass,
+ * fp32 intermediate, height pass) -> out = resized * a_c + b_c -> zero pad -> fp32 NCHW [B,3,S,S].  Replaces the loaders'
+ * pil_to_tensor -> ResizeLongestSide.apply_image_torch -> norm -> pad (stage1/data/sa1b_dataset.py:68-69, 163-171, 216-227,
+ * coco_dataset.py:146-153, transforms.py:48-54) and SAM2Transforms' ToTensor -> Resize((S,S)) -> Normalize (sam1_utils.py:17-41).
+ * table: [B][16] int64 on the device, one descriptor per image: {device address, element strides of channel / row / column,
+ * in_h, in_w, out_h, out_w (<= S), dtype (0 uint8, 1 fp32), staged planes (1 interleaved, 3 planar), input columns per staging
+ * chunk, taps per output along x / y, offsets (floats) of the x / y tap records in `taps`, unused}.  affine: [B][6] fp32
+ * (a_0..2, b_0..2).  taps: fp32 workspace of (K + 2) floats per output coordinate and axis.  max_out: largest out_h / out_w.
+ * Two kernels: tap tables, then the fused resize. */
+int es3_preprocess_images(const long long* table, const float* affine, float* taps, int B, int S, int max_out, float* out,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif
